@@ -232,6 +232,14 @@ def agent_train_timing(dev, pop, n_envs, generations=6, prefetch=True):
     return float(np.median(gaps)), stats, ag
 
 
+def dump_outputs(out_dir, res, fit_all):
+    """What the last timed step handed its caller: per-trajectory returns and executed steps of this rank's population
+    [pop, n_envs] and the gathered per-actor fitness [pop_total], as float64 .npy files (1.05 MB at the bench size)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (('returns', res.returns), ('steps', res.steps), ('fitness', fit_all)):
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().cpu().numpy().astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -285,7 +293,7 @@ def run_ours(args):
                 'md': md_host.to(dev), 'order': rollout.variant_sorted_order(md_host.to(dev)), 'pop_total': POP if shard else POP * world}
 
     def make_step(wl):
-        fit_all = torch.empty((wl['pop_total'],), dtype=torch.float64, device=dev)
+        fit_all = wl['fit_all'] = torch.empty((wl['pop_total'],), dtype=torch.float64, device=dev)
 
         def one_step(res=None):
             r = rollout.population_rollout(wl['w'], sh, wl['lv'], wl['st'], wl['md'], horizon=HORIZON, out=res, env_order=wl['order'])
@@ -314,6 +322,8 @@ def run_ours(args):
     clocks = sampler.stop() if sampler else None
     launches = (_native.lib().serl_launch_count() - launches0) // (args.steps + args.warmup) * args.steps
     res = m['res']
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, wl['fit_all'])
 
     # ---- end to end through the public API with host buffers (H2D genomes + env params, D2H fitness) every step
     pop_local = wl['w'].shape[0]
@@ -499,9 +509,13 @@ def main():
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-generation', action='store_true', help='skip the rollout+epoch generation timing and the other-workload legs')
     ap.add_argument('--no-agent', action='store_true', help='skip the Agent.train() timing')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the returns, executed steps and gathered fitness of the last timed step to DIR/<name>.npy (CUDA arm only)')
     ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                     help='weak: BASELINE config 3 per GPU (pop=512/GPU); strong: BASELINE config 4 (ONE pop=512, mixed faults, sharded)')
     args = ap.parse_args()
+    if args.impl == 'reference' and args.dump_outputs:
+        ap.error('--dump-outputs writes what the CUDA path computed; the reference arm only measures throughput')
     if args.impl == 'reference':
         run_reference(args)
     else:

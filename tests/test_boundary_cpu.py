@@ -10,11 +10,10 @@ import torch.multiprocessing as mp
 from oracle import actor as OA
 
 
-def make_args(pop=4, hidden=8):
+def make_args(folder, pop=4, hidden=8):
     from serl_b200.parameters import Parameters
     cla = types.SimpleNamespace(env='PHlab_attitude_nominal', seed=7, pop_size=pop, mut_type='normal')
-    os.makedirs('/tmp/serl_test', exist_ok=True)
-    cwd = os.getcwd(); os.chdir('/tmp/serl_test')
+    cwd = os.getcwd(); os.chdir(folder)          # Parameters creates ./tmp/ for checkpoints
     try:
         args = Parameters(cla)
     finally:
@@ -24,9 +23,9 @@ def make_args(pop=4, hidden=8):
     return args
 
 
-def test_population_views_and_reference_init_order():
+def test_population_views_and_reference_init_order(tmp_path):
     from serl_b200.population import PopulationList
-    args = make_args()
+    args = make_args(tmp_path)
     torch.manual_seed(7)
     pop = PopulationList(args, device='cpu')
     torch.manual_seed(7)
@@ -44,9 +43,9 @@ def test_population_views_and_reference_init_order():
     assert pop[0].actor.select_action(obs).shape == (3,)
 
 
-def test_ssne_rejects_out_of_scope_operators():
+def test_ssne_rejects_out_of_scope_operators(tmp_path):
     from serl_b200.core.mod_neuro_evo import SSNE
-    args = make_args()
+    args = make_args(tmp_path)
     args.mut_type = 'proximal'
     assert SSNE(args, None, None).mutate == 'proximal'        # batched on the device (serl_b200/evo_prox.py)
     args.distil_crossover, args.distil_type = True, 'fitness'

@@ -13,16 +13,16 @@ from oracle import actor as OA, phlab, plant as OP
 pytestmark = pytest.mark.gpu
 
 
-def make_args(pop=6, hidden=16, **kw):
+def make_args(folder, pop=6, hidden=16, **kw):
     from serl_b200.parameters import Parameters
     cla = types.SimpleNamespace(env='PHlab_attitude_nominal', seed=7, pop_size=pop, mut_type='normal', test_ea=True, **kw)
-    os.makedirs('/tmp/serl_test', exist_ok=True)
-    cwd = os.getcwd(); os.chdir('/tmp/serl_test')
+    os.makedirs(folder, exist_ok=True)
+    cwd = os.getcwd(); os.chdir(folder)
     try:
         args = Parameters(cla)
     finally:
         os.chdir(cwd)
-    args.save_foldername = '/tmp/serl_test/'
+    args.save_foldername = str(folder) + '/'
     args.state_dim, args.action_dim, args.hidden_size = 7, 3, hidden
     return args
 
@@ -55,39 +55,36 @@ def test_plant_step_kernel_matches_oracle(variant):
     assert np.allclose(got[:, live], ref[:, live], rtol=1e-11, atol=1e-12)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'citation_gust.so')),
-                    reason='needs the reference gust binary under oracle/_ref')
 @pytest.mark.parametrize('build', ['gust', 'test'])
 def test_timed_plant_step_api_flies_the_gust_pulse_like_the_binary(build):
     """serl_plant_step_timed with SERL_MODE_GUST (the per-step path of CitationEnv in 'gust' mode): one-step predictions from
-    the binary's own states through both edges of the pulse (native calls 1996..2003, 2296..2303) and in its middle."""
+    the binary's own states through both edges of the pulse (native calls 1996..2003, 2296..2303) and in its middle.  The
+    binary's states before and after those calls are recorded in tests/golden/refbin_kat.npz (envs/test: the same pulse with
+    the opposite sign)."""
     from serl_b200 import _native, rollout
     L = _native.lib()
     dev = torch.device('cuda:0')
     st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-    pl = OP.RefPlant(build)          # envs/test: the same pulse with the opposite sign
-    X = pl.initial_state()
+    kat = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'refbin_kat.npz'))
     var = torch.tensor([rollout.mode_code(build) & ~0xff00], dtype=torch.int32, device=dev)
     live = [0, 1, 2, 3, 4, 5, 6, 7, 9, 12, 15, 16, 17, 18]
     worst, changed = 0.0, 0
-    for k in range(2306):
+    window = [k for k in range(2306) if 1996 <= k <= 2003 or 2296 <= k <= 2303 or k == 2150]
+    assert kat[build + '_k'].tolist() == window
+    for k, X0, X in zip(window, kat[build + '_X0'], kat[build + '_X1']):
         cmd = 0.02 * np.sin(0.01 * k + np.arange(3))
-        window = 1996 <= k <= 2003 or 2296 <= k <= 2303 or k == 2150
-        if window:
-            Xd = torch.as_tensor(X[None].copy(), device=dev)
-            d = torch.as_tensor(cmd[None].copy(), device=dev)
-            call = torch.tensor([k], dtype=torch.int32, device=dev)
-            _native.check(L.serl_plant_step_timed(ctypes.c_void_p(Xd.data_ptr()), ctypes.c_void_p(d.data_ptr()), ctypes.c_void_p(var.data_ptr()),
-                                                  ctypes.c_void_p(call.data_ptr()), 1, st), 'serl_plant_step_timed')
-            call0 = torch.tensor([0], dtype=torch.int32, device=dev)
-            Xn = torch.as_tensor(X[None].copy(), device=dev)
-            _native.check(L.serl_plant_step_timed(ctypes.c_void_p(Xn.data_ptr()), ctypes.c_void_p(d.data_ptr()), ctypes.c_void_p(var.data_ptr()),
-                                                  ctypes.c_void_p(call0.data_ptr()), 1, st), 'serl_plant_step_timed')
-        _, X = pl.step(X, np.concatenate([cmd, np.zeros(7)]))
-        if window:
-            got = Xd.cpu().numpy()[0]
-            worst = max(worst, np.abs(got[live] - X[live]).max())
-            changed += int(np.abs(Xn.cpu().numpy()[0][live] - X[live]).max() > 1e-6)        # the same step outside the pulse (call 0)
+        Xd = torch.as_tensor(X0[None].copy(), device=dev)
+        d = torch.as_tensor(cmd[None].copy(), device=dev)
+        call = torch.tensor([k], dtype=torch.int32, device=dev)
+        _native.check(L.serl_plant_step_timed(ctypes.c_void_p(Xd.data_ptr()), ctypes.c_void_p(d.data_ptr()), ctypes.c_void_p(var.data_ptr()),
+                                              ctypes.c_void_p(call.data_ptr()), 1, st), 'serl_plant_step_timed')
+        call0 = torch.tensor([0], dtype=torch.int32, device=dev)
+        Xn = torch.as_tensor(X0[None].copy(), device=dev)
+        _native.check(L.serl_plant_step_timed(ctypes.c_void_p(Xn.data_ptr()), ctypes.c_void_p(d.data_ptr()), ctypes.c_void_p(var.data_ptr()),
+                                              ctypes.c_void_p(call0.data_ptr()), 1, st), 'serl_plant_step_timed')
+        got = Xd.cpu().numpy()[0]
+        worst = max(worst, np.abs(got[live] - X[live]).max())
+        changed += int(np.abs(Xn.cpu().numpy()[0][live] - X[live]).max() > 1e-6)        # the same step outside the pulse (call 0)
     assert worst < 1e-9, worst
     assert changed >= 10
 
@@ -109,10 +106,10 @@ def test_citation_env_step_api_matches_oracle_env():
     assert abs(info['t'] - o_info['t']) < 1e-12
 
 
-def test_agent_evaluate_returns_reference_shaped_episode():
+def test_agent_evaluate_returns_reference_shaped_episode(tmp_path):
     from serl_b200.core import agent as agent_mod
     from serl_b200.envs import config
-    args = make_args(pop=4, hidden=72)
+    args = make_args(tmp_path, pop=4, hidden=72)
     env = config.select_env('PHlab_attitude_nominal')
     torch.manual_seed(7); np.random.seed(7); random.seed(7)
     ag = agent_mod.Agent(args, env)
@@ -139,10 +136,10 @@ def test_agent_evaluate_returns_reference_shaped_episode():
     assert len(ag.replay_buffer) == n and ag.num_frames == n
 
 
-def test_agent_train_generations_and_checkpoint_format():
+def test_agent_train_generations_and_checkpoint_format(tmp_path):
     from serl_b200.core import agent as agent_mod
     from serl_b200.envs import config
-    args = make_args(pop=6, hidden=16)
+    args = make_args(tmp_path, pop=6, hidden=16)
     env = config.select_env('PHlab_attitude_nominal')
     torch.manual_seed(7); np.random.seed(7); random.seed(7)
     ag = agent_mod.Agent(args, env)
@@ -158,17 +155,17 @@ def test_agent_train_generations_and_checkpoint_format():
     assert ag.num_frames > 0 and ag.num_episodes > 0
     assert set(ag.evolver.selection_stats) == {'elite', 'selected', 'discarded', 'total'} and ag.evolver.selection_stats['total'] >= 1
     ag.save_agent(args, stats['elite_index'])
-    pop_dict = torch.load('/tmp/serl_test/evo_nets.pkl', weights_only=False)
+    pop_dict = torch.load(os.path.join(args.save_foldername, 'evo_nets.pkl'), weights_only=False)
     assert sorted(pop_dict) == ['actor_%d' % i for i in range(6)]
     assert list(pop_dict['actor_0'])[:2] == ['net.0.weight', 'net.0.bias']
-    oracle_actor = OA.from_state_dict(torch.load('/tmp/serl_test/elite_net.pkl', weights_only=False), 'tanh')   # loads into the reference layout
+    oracle_actor = OA.from_state_dict(torch.load(os.path.join(args.save_foldername, 'elite_net.pkl'), weights_only=False), 'tanh')   # loads into the reference layout
     assert np.array_equal(OA.flatten(oracle_actor), ag.pop.genomes[int(stats['elite_index'])].cpu().numpy())
 
 
-def _train_generations(prefetch, n, poke=None):
+def _train_generations(folder, prefetch, n, poke=None):
     from serl_b200.core import agent as agent_mod
     from serl_b200.envs import config
-    args = make_args(pop=6, hidden=16)
+    args = make_args(folder, pop=6, hidden=16)
     args.prefetch_generation = prefetch
     env = config.select_env('PHlab_attitude_nominal')
     torch.manual_seed(7); np.random.seed(7); random.seed(7)
@@ -184,11 +181,11 @@ def _train_generations(prefetch, n, poke=None):
     return out, flags, ag
 
 
-def test_next_generation_front_launched_ahead_changes_no_result():
+def test_next_generation_front_launched_ahead_changes_no_result(tmp_path):
     """train() queues the next generation's rollouts before waiting for its own validation scores; the statistics of
     every generation, the populations and the counters must equal those of strictly one generation per call."""
-    a, fa, aga = _train_generations(True, 3)
-    b, fb, agb = _train_generations(False, 3)
+    a, fa, aga = _train_generations(tmp_path / 'a', True, 3)
+    b, fb, agb = _train_generations(tmp_path / 'b', False, 3)
     assert fa == [0.0, 1.0, 1.0] and fb == [0.0, 0.0, 0.0]
     for x, y in zip(a, b):
         for k in x:
@@ -198,8 +195,8 @@ def test_next_generation_front_launched_ahead_changes_no_result():
     assert len(aga.replay_buffer) == len(agb.replay_buffer)
 
 
-def test_front_launched_ahead_is_dropped_when_the_population_changed():
-    a, fa, _ = _train_generations(True, 3, poke=1)
+def test_front_launched_ahead_is_dropped_when_the_population_changed(tmp_path):
+    a, fa, _ = _train_generations(tmp_path, True, 3, poke=1)
     assert fa == [0.0, 0.0, 1.0]
     assert all(np.isfinite(s['best_train_fitness']) for s in a)
 

@@ -10,6 +10,7 @@ from oracle import actor as A, phlab, refsig
 
 pytestmark = pytest.mark.gpu
 ACT = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'actors.npz'))
+REFBIN = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'refbin_kat.npz'))
 
 
 class KOActor:
@@ -109,12 +110,11 @@ def test_noise_mode_and_time_triggered_modes_are_named():
         config.select_env('PHlab_attitude_nosuchmode')
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'citation_cg_timed.so')),
-                    reason='needs the reference cg_timed binary under oracle/_ref')
 def test_cg_timed_build_switches_at_20_s_like_the_reference_binary():
     """envs/cg_timed ('CG Aft after 20s', envs/phlabenv.py:159-163): nominal dynamics until the model clock reaches 20 s — in the
     LAST ode5 stage of native call 1999 — then three moment-arm parameters change.  40 s episodes (4001 steps) through the
-    kernel vs the reference binary stepped by the oracle env; also the plain cg and nominal modes must differ from it."""
+    kernel vs the reference binary stepped by the oracle env (recorded by tests/golden/make_golden_refbin.py: live states every
+    20th step and around the switch, executed steps, return); also the plain cg and nominal modes must differ from it."""
     from serl_b200 import rollout
     dev = torch.device('cuda:0')
     g = ACT['serl10_elite_h72_tanh']
@@ -125,33 +125,23 @@ def test_cg_timed_build_switches_at_20_s_like_the_reference_binary():
     r = run('cg-timed')
     torch.cuda.synchronize()
     r.check()
-    env = phlab.CitationEnv('cg-timed', 'ref', t_max=40)
-    env.smooth_w = 6.0
-    obs = env.reset(lv[0], st[0])
-    tot, xs = 0.0, []
-    for k in range(4001):
-        obs, rew, done, _ = env.step(KOActor(g).select_action(obs))
-        xs.append(env.x.copy())
-        tot += rew
-        if done:
-            break
-    assert int(r.steps[0, 0]) == k + 1 == 4001
-    tx = r.trace_x[0, 0, :k + 1].cpu().numpy()
+    n, tot, rows = int(REFBIN['cg_timed_steps']), float(REFBIN['cg_timed_return']), REFBIN['cg_timed_rows']
+    assert int(r.steps[0, 0]) == n == 4001
+    tx = r.trace_x[0, 0, :n].cpu().numpy()
     live = [0, 1, 2, 3, 4, 5, 6, 7, 9]
-    assert np.abs(tx[:, live] - np.asarray(xs)[:, live]).max() < 1e-8
+    assert np.abs(tx[rows][:, live] - REFBIN['cg_timed_x']).max() < 1e-8
     assert abs(float(r.returns[0, 0]) - tot) <= 1e-8 * abs(tot)
     nominal = run('nominal')
     assert np.array_equal(nominal.trace_x[0, 0, :1999].cpu().numpy()[:, live], tx[:1999, live])        # identical before the trigger
     assert np.abs(nominal.trace_x[0, 0, 2100:2400].cpu().numpy()[:, live] - tx[2100:2400, live]).max() > 1e-5
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'citation_gust.so')),
-                    reason='needs the reference gust binary under oracle/_ref')
 def test_gust_build_flies_the_pulse_like_the_reference_binary():
     """envs/gust ('Vertical Gust of 15ft/s at 20s', envs/phlabenv.py:165-169): nominal dynamics, and for 20 s <= t <= 23 s the
     aerodynamic angle of attack is alpha - atan(w / V).  A 30 s episode (3001 steps, sensor noise off) through the kernel vs the
-    reference binary stepped by the oracle env; the untraced launch (stage derivatives in tensor memory) must return the same bits
-    as the traced one (local memory)."""
+    reference binary stepped by the oracle env (recorded by tests/golden/make_golden_refbin.py: live states every 20th step and
+    around both edges of the pulse, executed steps, return); the untraced launch (stage derivatives in tensor memory) must
+    return the same bits as the traced one (local memory)."""
     from serl_b200 import rollout
     dev = torch.device('cuda:0')
     g = ACT['serl10_elite_h72_tanh']
@@ -163,21 +153,12 @@ def test_gust_build_flies_the_pulse_like_the_reference_binary():
     r = run('gust', True)
     torch.cuda.synchronize()
     r.check()
-    env = phlab.CitationEnv('gust', 'ref', t_max=30)
-    env.smooth_w = 4.5
-    obs = env.reset(lv[0], st[0])
-    tot, xs = 0.0, []
-    for k in range(3001):
-        obs, rew, done, _ = env.step(KOActor(g).select_action(obs))
-        xs.append(env.x.copy())
-        tot += rew
-        if done:
-            break
-    assert int(r.steps[0, 0]) == k + 1
-    tx = r.trace_x[0, 0, :k + 1].cpu().numpy()
+    n, tot, rows = int(REFBIN['gust_steps']), float(REFBIN['gust_return']), REFBIN['gust_rows']
+    assert int(r.steps[0, 0]) == n
+    tx = r.trace_x[0, 0, :n].cpu().numpy()
     live = [0, 1, 2, 3, 4, 5, 6, 7, 9]
-    err = np.abs(tx[:, live] - np.asarray(xs)[:, live]).max(axis=1)
-    assert err.max() < 1e-8, (int(err.argmax()), float(err.max()), err[1995:2005], err[2295:2305])
+    err = np.abs(tx[rows][:, live] - REFBIN['gust_x']).max(axis=1)
+    assert err.max() < 1e-8, (int(rows[err.argmax()]), float(err.max()))
     assert abs(float(r.returns[0, 0]) - tot) <= 1e-8 * abs(tot)
     nominal = run('nominal', True)
     assert np.array_equal(nominal.trace_x[0, 0, :1999].cpu().numpy()[:, live], tx[:1999, live])        # identical before the gust

@@ -1,16 +1,15 @@
 """N3: proximal / safe mutation batched over the population (serl_b200/evo_prox.py) against (a) the reference module itself
-(base/core/mod_neuro_evo.py:183-252, imported in the build container) and (b) a per-actor autograd restatement."""
+(base/core/mod_neuro_evo.py:183-252, results recorded in tests/golden/refbin_kat.npz) and (b) a per-actor autograd restatement."""
+import hashlib
 import os
-import sys
-import types
 
 import numpy as np
-import pytest
 import torch
 
+from oracle import actor as OA
 from serl_b200 import evo, evo_prox
 
-REF = '/root/reference/base'
+KAT = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'refbin_kat.npz'))
 
 
 def per_actor_reference(genome, states, shape, activation, mag, delta):
@@ -50,86 +49,55 @@ def test_batched_equals_per_actor_restatement():
     assert torch.equal(G2[:, ~m], G[:, ~m])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='needs the reference tree (build container only)')
-def test_batched_proximal_mutation_equals_the_reference_module(tmp_path, monkeypatch):
-    monkeypatch.chdir(tmp_path)
-    saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == 'core' or k.startswith('core.') or k == 'parameters'}
-    sys.path.insert(0, REF)
-    try:
-        from core import mod_neuro_evo as ref_ne, genetic_agent as ref_ga
-        from parameters import Parameters as RefP
-        import torch.distributions as dist
-        args = RefP(types.SimpleNamespace(pop_size=4, mut_type='proximal', env='x', frames=1, seed=1, disable_cuda=True))
-        args.state_dim, args.action_dim, args.device = 7, 3, torch.device('cpu')
-        torch.manual_seed(0)
-        genes = [ref_ga.GeneticAgent(args) for _ in range(3)]
-        shape = (7, 3, args.hidden_size, args.num_layers)
-        G = torch.stack([torch.cat([p.data.reshape(-1) for p in g.actor.parameters()]) for g in genes])
-        states = torch.randn(3, 32, 7) * 0.1
-        ssne = ref_ne.SSNE(args, None, None)
+def reference_init(n):
+    """n flat genomes drawn by the oracle's Actor (the reference's layer order and init draws) under the current torch seed."""
+    return torch.from_numpy(np.stack([OA.flatten(OA.Actor()) for _ in range(n)]))
 
-        class FakeBuf:
-            def __init__(self, st):
-                self.st = st
 
-            def __len__(self):
-                return 32
+def check_reference_start(G, key):
+    """the rebuilt starting genomes must be the reference's own: SHA-256 of their float32 bytes, recorded by
+    tests/golden/make_golden_refbin.py."""
+    digest = hashlib.sha256(np.ascontiguousarray(G.numpy(), dtype=np.float32).tobytes()).hexdigest()
+    assert digest == str(KAT[key]), "the rebuilt starting genomes differ from the reference's: oracle.actor.Actor no longer draws like it"
 
-            def sample(self, n):
-                return (self.st, None, None, None, None)
-        deltas = []
-        for k, g in enumerate(genes):
-            g.buffer = FakeBuf(states[k])
-            tot = g.actor.count_parameters()
-            torch.manual_seed(100 + k)
-            deltas.append(dist.Normal(torch.zeros(tot), torch.ones(tot) * args.mutation_mag).sample())
-            torch.manual_seed(100 + k)
-            ssne.proximal_mutate(g, mag=args.mutation_mag)
-        G_ref = torch.stack([torch.cat([p.data.reshape(-1) for p in g.actor.parameters()]) for g in genes])
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == 'core' or k.startswith('core.') or k == 'parameters']:
-            del sys.modules[k]
-        sys.modules.update(saved)
+
+def test_batched_proximal_mutation_equals_the_reference_module():
+    """reference: SSNE.proximal_mutate (base/core/mod_neuro_evo.py:183-252) on three seeded actors, recorded at fixed
+    genome coordinates by tests/golden/make_golden_refbin.py."""
+    import torch.distributions as dist
+    torch.manual_seed(0)
+    G = reference_init(3)
+    check_reference_start(G, 'proximal_G_init_sha256')
+    shape = (7, 3, 72, 3)
+    states = torch.randn(3, 32, 7) * 0.1
+    mag = float(KAT['mutation_mag'])
+    tot = int(evo_prox.weight_mask(shape, G.device).sum())          # Actor.count_parameters(): the 2-D weights
+    deltas = []
+    for k in range(3):
+        torch.manual_seed(100 + k)
+        deltas.append(dist.Normal(torch.zeros(tot), torch.ones(tot) * mag).sample())
     G2 = G.clone()
-    evo_prox.proximal_mutate_batched(G2, [0, 1, 2], states, shape, args.activation_actor, args.mutation_mag, delta=torch.stack(deltas))
-    assert (G_ref - G).abs().max() > 0.1
-    assert (G2 - G_ref).abs().max().item() <= 1e-6
+    evo_prox.proximal_mutate_batched(G2, [0, 1, 2], states, shape, 'tanh', mag, delta=torch.stack(deltas))
+    cols = torch.as_tensor(KAT['genome_sample'], dtype=torch.long)
+    G_ref = torch.as_tensor(KAT['proximal_G_ref'])
+    assert (G_ref - G[:, cols]).abs().max() > 0.1
+    assert (G2[:, cols] - G_ref).abs().max().item() <= 1e-6
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='needs the reference tree (build container only)')
-def test_batched_distillation_step_equals_the_reference_update_parameters(tmp_path, monkeypatch):
-    """one Q-filtered behaviour-cloning Adam step (base/core/genetic_agent.py:22-60) for three children at once."""
+def test_batched_distillation_step_equals_the_reference_update_parameters():
+    """one Q-filtered behaviour-cloning Adam step (base/core/genetic_agent.py:22-60) for three children at once; reference
+    genomes and losses recorded by tests/golden/make_golden_refbin.py."""
     from serl_b200 import evo_distil
-    monkeypatch.chdir(tmp_path)
-    saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == 'core' or k.startswith('core.') or k == 'parameters'}
-    sys.path.insert(0, REF)
-    try:
-        from core import genetic_agent as ref_ga
-        from parameters import Parameters as RefP
-        args = RefP(types.SimpleNamespace(pop_size=4, mut_type='proximal', env='x', frames=1, seed=1, disable_cuda=True))
-        args.state_dim, args.action_dim, args.device = 7, 3, torch.device('cpu')
-        torch.manual_seed(0)
-        kids = [ref_ga.GeneticAgent(args) for _ in range(3)]
-        p1s = [ref_ga.GeneticAgent(args) for _ in range(3)]
-        p2s = [ref_ga.GeneticAgent(args) for _ in range(3)]
-        flat = lambda g: torch.cat([p.data.reshape(-1) for p in g.actor.parameters()])
-        lin = torch.nn.Linear(10, 2)
+    torch.manual_seed(0)
+    G0, G1, G2 = reference_init(3), reference_init(3), reference_init(3)
+    check_reference_start(torch.cat([G0, G1, G2]), 'distil_G_init_sha256')
+    lin = torch.nn.Linear(10, 2)
 
-        def critic(s, a):
-            q = lin(torch.cat((s, a), 1))
-            return q[:, :1], q[:, 1:]
-        states = torch.randn(3, 40, 7) * 0.2
-        shape = (7, 3, args.hidden_size, args.num_layers)
-        G0 = torch.stack([flat(k) for k in kids])
-        G1, G2 = torch.stack([flat(p) for p in p1s]), torch.stack([flat(p) for p in p2s])
-        mse_ref = [kids[c].update_parameters((states[c], None, None, None, None), p1s[c].actor, p2s[c].actor, critic) for c in range(3)]
-        G_ref = torch.stack([flat(k) for k in kids])
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == 'core' or k.startswith('core.') or k == 'parameters']:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    def critic(s, a):
+        q = lin(torch.cat((s, a), 1))
+        return q[:, :1], q[:, 1:]
+    states = torch.randn(3, 40, 7) * 0.2
+    shape = (7, 3, 72, 3)
     child = G0.clone().requires_grad_(True)
     opt = torch.optim.Adam([child], lr=1e-3)
     with torch.no_grad():
@@ -142,9 +110,11 @@ def test_batched_distillation_step_equals_the_reference_update_parameters(tmp_pa
     loss, mse = evo_distil.cloning_loss(evo_prox.actor_forward_batched(child, states, shape, 'tanh'), a1, a2, q1, q2)
     loss.backward()
     opt.step()
-    assert (G_ref - G0).abs().max() > 1e-4
-    assert (child.detach() - G_ref).abs().max().item() <= 2e-6
-    assert np.allclose(mse.numpy(), np.asarray(mse_ref), rtol=1e-4)
+    cols = torch.as_tensor(KAT['genome_sample'], dtype=torch.long)
+    G_ref = torch.as_tensor(KAT['distil_G_ref'])
+    assert (G_ref - G0[:, cols]).abs().max() > 1e-4
+    assert (child.detach()[:, cols] - G_ref).abs().max().item() <= 2e-6
+    assert np.allclose(mse.numpy(), KAT['distil_mse_ref'], rtol=1e-4)
 
 
 def test_sort_groups_by_fitness_order():

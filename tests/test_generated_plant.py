@@ -1,7 +1,7 @@
 """The GENERATED device sources (serl_b200/csrc/gen: fast mode, merged variants, pooled constants, table blob) are
 checked on the CPU: compiled with gcc behind trivial macro definitions and compared with the oracle's exact restatement on
-the reference-recorded right-hand-side vectors.  Also: the committed generated files are reproducible from the reference
-binaries (container only)."""
+the reference-recorded right-hand-side vectors and the gust / test binaries' recorded states (tests/golden).  Also: the
+committed generated files are reproducible from the reference binaries' byte copies under oracle/_ref (oracle/build.py)."""
 import ctypes
 import os
 import subprocess
@@ -12,6 +12,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 KAT = np.load(os.path.join(ROOT, 'tests', 'golden', 'plant_rhs_kat.npz'))
+REFBIN = np.load(os.path.join(ROOT, 'tests', 'golden', 'refbin_kat.npz'))
 VARIANTS = ['h2000_v90', 'ice', 'cg', 'cg_for', 'h2000_v150', 'h10000_v90']
 LIVE = [0, 1, 2, 3, 4, 5, 6, 7, 9, 12, 15, 16, 17, 18]
 
@@ -96,25 +97,18 @@ def test_generated_device_rhs_matches_reference_binary_vectors(devlib, variant):
     assert worst < (5e-4 if which == 'gen_f32' else 1e-11), worst
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/envs'), reason='needs the reference tree (build container only)')
 @pytest.mark.parametrize('build,sign', [('gust', 1.0), ('test', -1.0)])
-def test_gust_build_is_the_nominal_rhs_with_an_angle_of_attack_offset(devlib, tmp_path, build, sign):
+def test_gust_build_is_the_nominal_rhs_with_an_angle_of_attack_offset(devlib, build, sign):
     """envs/gust ("vertical gust of 15 ft/s at 20 s"): ode5 over the generated right-hand side with U[3] = atan(w / V) for the
     stages inside 20 s <= t <= 23 s (last stage of native call 1999, calls 2000..2299, first stage of call 2300) reproduces
     the gust BINARY bit for bit (reference-order build) through both edges of the pulse.  envs/test is the same pulse with the
-    opposite sign (U[3] = -atan(w / V))."""
+    opposite sign (U[3] = -atan(w / V)).  The binary's states before and after those calls, stepped from initialize() with
+    cmd = 0.02 sin(0.01 k + [0, 1, 2]), are recorded in tests/golden/refbin_kat.npz."""
     import math
-    import shutil
     which, lib = devlib
     if which == 'gen_f32':
         pytest.skip('double-precision check')
     D = ctypes.c_double
-    so = tmp_path / 'gust.so'
-    shutil.copy('/root/reference/envs/%s/_citation.cpython-38-x86_64-linux-gnu.so' % build, so)
-    ref = ctypes.CDLL(str(so))
-    ref.step.argtypes = [ctypes.POINTER(D), ctypes.POINTER(D)]
-    ref.initialize()
-    rtx = (D * 19).in_dll(ref, 'rtX')
     B = [[1 / 5, 0, 0, 0, 0, 0], [3 / 40, 9 / 40, 0, 0, 0, 0], [44 / 45, -56 / 15, 32 / 9, 0, 0, 0],
          [19372 / 6561, -25360 / 2187, 64448 / 6561, -212 / 729, 0, 0], [9017 / 3168, -355 / 33, 46732 / 5247, 49 / 176, -5103 / 18656, 0],
          [35 / 384, 0, 500 / 1113, 125 / 192, -2187 / 6784, 11 / 84]]
@@ -138,32 +132,36 @@ def test_gust_build_is_the_nominal_rhs_with_an_angle_of_attack_offset(devlib, tm
                     acc += f[j][i] * (h * B[s][j])
                 x[i] = X[i] + acc
         return x
-    cmd, out = (D * 10)(), (D * 12)()
-    X = np.array(rtx[:])
     worst, active = 0.0, 0
-    for k in range(2306):
+    window = [k for k in range(2306) if 1996 <= k <= 2003 or 2296 <= k <= 2303 or k == 2150]
+    assert REFBIN[build + '_k'].tolist() == window
+    for k, X, Xb in zip(window, REFBIN[build + '_X0'], REFBIN[build + '_X1']):
         c = 0.02 * np.sin(0.01 * k + np.arange(3))
-        cmd[0], cmd[1], cmd[2] = c
-        window = 1996 <= k <= 2003 or 2296 <= k <= 2303 or k == 2150
-        Xn = step(X, c, k) if window else None
-        ref.step(cmd, out)
-        Xb = np.array(rtx[:])
-        if window:
-            err = np.abs(Xn[idx] - Xb[idx]).max()
-            worst = max(worst, err / np.abs(Xb[idx]).max())
-            if which == 'gen_exact':
-                assert err == 0.0, (k, err)
-            nominal = step(X, c, -1)
-            active += int(np.abs(nominal[idx] - Xb[idx]).max() > 0)
-        X = Xb
+        Xn = step(X, c, k)
+        err = np.abs(Xn[idx] - Xb[idx]).max()
+        worst = max(worst, err / np.abs(Xb[idx]).max())
+        if which == 'gen_exact':
+            assert err == 0.0, (k, err)
+        nominal = step(X, c, -1)
+        active += int(np.abs(nominal[idx] - Xb[idx]).max() > 0)
     assert worst < 1e-12 and active >= 10        # fast build: <= 1 ulp per operation; the gust really is on in the window
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/envs'), reason='needs the reference tree (build container only)')
+def _have_ref_binaries():
+    from oracle import build as obuild
+    return all(os.path.exists(os.path.join(obuild.HERE, '_ref', 'citation_%s.so' % v)) for v in obuild.VARIANTS + obuild.REF_ONLY)
+
+
+@pytest.mark.skipif(not _have_ref_binaries(), reason='needs the reference plant binaries under oracle/_ref (oracle/build.py)')
 def test_committed_generated_sources_are_reproducible(tmp_path):
-    """tools/lift regenerates byte-identical device sources from the reference binaries."""
-    code = ("import sys, os; sys.path.insert(0, %r); import gen_all as G; G.emit_set(%r, live=True)" %
-            (os.path.join(ROOT, 'tools', 'lift'), str(tmp_path / 'gen')))
+    """tools/lift regenerates byte-identical device sources from the reference binaries (oracle/_ref); the lifter's working
+    copies of the binaries go to tmp_path."""
+    code = ("import sys; sys.path.insert(0, %r); import gen_plant, gen_all as G, symtrace as S; "
+            "gen_plant.REF = %r; init = S.Image.__init__; "
+            "S.Image.__init__ = lambda self, so, workdir: init(self, so, %r); "
+            "G.emit_set(%r, live=True)" %
+            (os.path.join(ROOT, 'tools', 'lift'), os.path.join(ROOT, 'oracle', '_ref', 'citation_%s.so'), str(tmp_path / 'lift'),
+             str(tmp_path / 'gen')))
     subprocess.check_call([sys.executable, '-c', code], stdout=subprocess.DEVNULL)
     for f in sorted(os.listdir(tmp_path / 'gen')):
         a = open(tmp_path / 'gen' / f).read()
